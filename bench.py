@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--config C1|C2|C3|C4] [--mode fused|hll|counters|alive]
   python bench.py --impl reference --gpus N --steps K ...   the reference's CPU path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR    also writes the state the K timed steps computed as DIR/<name>.npy
 
 Workloads (BASELINE.json configs; SURVEY.md §8 d) — the default at every N is C1, per-GPU work fixed (weak scaling):
   C1  64 partitions, 1e8 messages per GPU, 256 B mean value, 16-byte keys, 1e7 distinct keys per GPU, 1 % null keys,
@@ -88,7 +89,13 @@ def parse():
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="skip the post-run parity check of the (merged) state")
     ap.add_argument("--cpu-sample", type=int, default=0, help="records in the CPU baseline sample (0 = auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the state they computed (what a caller reads back) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     c = CONFIGS[a.config]
     for k_arg, k_cfg in (("n", "n"), ("partitions", "partitions"), ("value_mean", "value_mean"), ("distinct_keys", "distinct_keys"),
                          ("tombstones", "tombstones"), ("null_keys", "nulls"), ("shard_world", "shard_world")):
@@ -306,6 +313,35 @@ def state_of(eng, P, mode):
     return s
 
 
+DUMP_PARTITIONS = 4096   # per-partition outputs of larger topics are dumped for a seeded sample of this many partitions
+
+
+def dump_outputs(eng, P, mode, out_dir, prefix=""):
+    """Writes the finalized state of the timed path, everything a caller reads back from it, as out_dir/<prefix><name>.npy,
+    so that two builds can be compared output for output on the same seeded topic.  Integer metrics are stored as float64
+    (exact below 2^53), the HLL registers as float32.  A topic with more than DUMP_PARTITIONS partitions is represented by
+    a fixed, seeded sample of them (partitions.npy names which), which keeps the files far below 64 MB."""
+    import numpy as np
+    parts = np.arange(P)
+    if P > DUMP_PARTITIONS:
+        parts = np.sort(np.random.default_rng(0).choice(P, DUMP_PARTITIONS, replace=False))
+    out = {"partitions": parts,
+           "counters": [[eng.counter(i, int(p)) for i in range(7)] for p in parts],
+           "key_size_hist": [eng.hist(0, int(p)) for p in parts],
+           "value_size_hist": [eng.hist(1, int(p)) for p in parts],
+           "globals": [eng.global_(i) for i in range(4)],
+           "timestamps": list(eng.timestamps())}
+    if mode in ("fused", "alive"):
+        out["alive_keys"] = [eng.alive_keys()]
+    if mode in ("fused", "hll"):
+        out["hll_registers"] = eng.hll_registers()
+        out["alive_keys_hll"] = [eng.alive_keys_hll()]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"),
+                np.asarray(v, dtype=np.float32 if name == "hll_registers" else np.float64))
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
@@ -341,7 +377,7 @@ def run_ours(a):
         dist.destroy_process_group()
 
 
-def measure(a, ctx, full):
+def measure(a, ctx, full, dump_prefix=""):
     torch, dist, kta, synth, allreduce_merge = ctx["torch"], ctx["dist"], ctx["kta"], ctx["synth"], ctx["merge"]
     rank, world, local, dev, barrier = ctx["rank"], ctx["world"], ctx["local"], ctx["dev"], ctx["barrier"]
     # ---- the rank's shard of the topic, generated in HBM ----
@@ -397,6 +433,8 @@ def measure(a, ctx, full):
     value = n_all * a.steps / (ms / 1e3)
     # sanity on the timed topic itself: K batches were counted (on every rank after the merge)
     assert eng.message_metrics.overall_count() == n_all * a.steps, (eng.message_metrics.overall_count(), n_all * a.steps)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(eng, P, a.mode, a.dump_outputs, dump_prefix)
     table = eng.alive_table_stats() if exact else None
 
     merge_ms = None
@@ -457,7 +495,7 @@ def measure(a, ctx, full):
 
     # ---- e2e: same metric through the host entry point, inputs in pinned host memory ----
     if not a.no_e2e:
-        e2e_steps = max(3, min(a.steps, 8))
+        e2e_steps = a.steps
         cols = {}
         for name in ("partition", "ts_ms", "key_len", "value_len", "key_tile_base"):
             src = getattr(topic, name)
@@ -603,7 +641,7 @@ def run_sweep(a, ctx):
     for vm in C4_VALUE_MEANS:
         b = argparse.Namespace(**vars(a))
         b.value_mean = vm
-        line = measure(b, ctx, full=False)
+        line = measure(b, ctx, full=False, dump_prefix="value_mean_%d_" % vm)
         points.append({"value_mean": vm, "value": line["value"], "ms_per_step": line["ms_per_step"],
                        "kernel_ms": line["roofline"]["kernel_ms"], "frac": line["roofline"]["frac"],
                        "logical_topic_gb_s": line["logical_topic_gb_s"]})
@@ -629,17 +667,17 @@ def extra_modes(a, topic, kta, torch, dev, peak):
                 for _ in range(k):
                     scan_topic(eng, topic, mode)
                 eng.finalize()
-            topic_pass(2)
+            topic_pass(max(1, a.warmup))
             eng.set_timing(True)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            topic_pass(5)
+            topic_pass(a.steps)
             e1.record()
             torch.cuda.synchronize(dev)
             kms, kn = eng.scan_time_ms()
             alg = 20 * topic.n + (topic.key_bytes_len if mode != "counters" else 0)
             ach = alg / (kms / kn / 1e3) / 1e9
-            out[mode] = {"msg_per_s": topic.n * 5 / (e0.elapsed_time(e1) / 1e3), "kernel_ms": kms / kn,
+            out[mode] = {"msg_per_s": topic.n * a.steps / (e0.elapsed_time(e1) / 1e3), "kernel_ms": kms / kn,
                          "achieved_gb_s": ach, "frac": ach / peak,
                          "alive_keys": eng.alive_keys() if mode in ("alive", "fused") else None}
             eng.close()
