@@ -206,8 +206,9 @@ int kta_alive_import_device(kta_handle *h, const uint32_t *dev_hash, const uint6
  * columns above (what librdkafka's parser + BorrowedMessage accessors do per message, src/kafka.rs:93,
  * src/metric.rs:208-209,218,233) and scans it.  Control batches are skipped, LogAppendTime batches use
  * maxTimestamp, a record's timestamp is baseTimestamp + timestampDelta (only a result of -1 is "not available"),
- * CRCs are not verified (librdkafka default check.crcs=false).  gzip, LZ4 (frame format) and Snappy (raw or
- * xerial-framed) batches are decompressed on the GPU; zstd batches are rejected (KTA_ERR_INVALID).
+ * CRCs are not verified (librdkafka default check.crcs=false).  gzip, LZ4 (frame format), Snappy (raw or
+ * xerial-framed) and zstd batches are decompressed on the GPU (zstd: no dictionaries; the content checksum is not
+ * verified); batches naming an unassigned codec (5-7) are rejected (KTA_ERR_INVALID).
  * Differences from a librdkafka consumer: records of aborted transactions ARE delivered (read_committed filtering
  * needs the transaction index, which is not read), legacy magic 0/1 message sets are reported as malformed. */
 /* raw bytes already in device memory; batch_off[nbatches] = byte offset of every batch header (device memory) */

@@ -5,8 +5,8 @@
 //               tombstone_per_10k=...,null_key_per_10k=...,zipf_keys=1,geometric_values=1
 //                                                                (the in-memory topic of BASELINE.json configs)
 //   --log-dir DIR              read Kafka log segments from DIR/<topic>-<partition>/*.log (a broker's data directory)
-//                              and decode them on the GPU (RecordBatch v2, magic 2; uncompressed, gzip, LZ4 or Snappy
-//                              batches; zstd is rejected).  Differences from a librdkafka
+//                              and decode them on the GPU (RecordBatch v2, magic 2; uncompressed, gzip, LZ4, Snappy or
+//                              zstd batches).  Differences from a librdkafka
 //                              consumer: records of ABORTED transactions are counted (a consumer with the default
 //                              isolation.level=read_committed filters them; the .txnindex files are not read here),
 //                              and legacy magic 0/1 message sets are reported as malformed.

@@ -730,15 +730,21 @@ static int scan_log_batches(kta_handle *h, int32_t partition, const int32_t *dev
     CU(cudaMemcpyAsync(err, h->d_log_err, 8, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     if (err[0] & LOGB_COMPRESSED)
-        return fail(KTA_ERR_INVALID, "zstd record batches are not supported (gzip, LZ4 and Snappy are decompressed on the GPU)");
+        return fail(KTA_ERR_INVALID, "unknown compression codec in a record batch of partition %d", partition);
     if (err[0] & LOGB_BAD) return fail(KTA_ERR_INVALID, "malformed record batch header in partition %d", partition);
     if (nrec == 0) return KTA_OK;
     if (err[0] & LOGB_CODECS) {
         // compressed batches: size pass, scratch allocation, decompression; afterwards they are ordinary batches that
         // happen to lie in the scratch buffer
+        const uint32_t codecs = err[0] & LOGB_CODECS;   // the codecs present (err[0] is reused by the size pass)
         if ((rc = grow(h->d_unc_slot, h->unc_slot_cap, nbatches + 2, s))) return rc;
         CU(cudaMemsetAsync(h->d_log_err, 0, 4, s));
         log_unc_size_kernel<<<grid, 128, 0, s>>>(dev_bytes, h->d_log_info, nbatches, h->d_unc_slot, h->d_log_err);
+        if (codecs & LOGB_ZSTD) {   // warp per batch
+            log_zstd_size_kernel<<<(int)std::min<int64_t>((nbatches + 3) / 4, (int64_t)h->sm_count * 16), 128, 0, s>>>(
+                dev_bytes, h->d_log_info, nbatches, h->d_unc_slot, h->d_log_err);
+            h->launches++;
+        }
         tile_base_scan_kernel<<<1, 1024, 0, s>>>(h->d_unc_slot, nbatches);
         CU(cudaGetLastError());
         h->launches += 2;
@@ -748,10 +754,16 @@ static int scan_log_batches(kta_handle *h, int32_t partition, const int32_t *dev
         CU(cudaStreamSynchronize(s));
         if (err[0]) return fail(KTA_ERR_INVALID, "malformed compressed record batch in partition %d", partition);
         if ((rc = grow(h->d_unc, h->unc_cap, (int64_t)unc_total + 64, s))) return rc;
-        log_decompress_kernel<<<(int)std::min<int64_t>((nbatches + 3) / 4, (int64_t)h->sm_count * 16), 128, 0, s>>>(
-            dev_bytes, h->d_log_info, nbatches, h->d_unc_slot, h->d_unc, h->d_log_err);
+        const int dgrid = (int)std::min<int64_t>((nbatches + 3) / 4, (int64_t)h->sm_count * 16);
+        if (codecs & ~LOGB_ZSTD) {
+            log_decompress_kernel<false><<<dgrid, 128, 0, s>>>(dev_bytes, h->d_log_info, nbatches, h->d_unc_slot, h->d_unc, h->d_log_err);
+            h->launches++;
+        }
+        if (codecs & LOGB_ZSTD) {
+            log_decompress_kernel<true><<<dgrid, 128, 0, s>>>(dev_bytes, h->d_log_info, nbatches, h->d_unc_slot, h->d_unc, h->d_log_err);
+            h->launches++;
+        }
         CU(cudaGetLastError());
-        h->launches++;
     }
     if ((int64_t)nrec >= ((int64_t)1 << 31) - 2) return fail(KTA_ERR_INVALID, "%llu records in one call: split the segments", (unsigned long long)nrec);
     const bool hash = h->need_hash || h->d_hash_out;

@@ -14,23 +14,26 @@
 // timestampDelta as the consumer computes it, and only a RESULT of -1 means "not available"; key/value length -1 means
 // null.  CRCs are not verified (librdkafka's default check.crcs=false).
 // Compression (attributes bits 0-2, librdkafka decompresses inside poll, src/kafka.rs:93): gzip (kta_inflate.cuh), LZ4 (frame
-// format) and Snappy (raw or xerial-framed) batches are decompressed on the GPU into a scratch buffer and then decoded like
-// the others; zstd is rejected.
+// format), Snappy (raw or xerial-framed) and zstd (kta_zstd.cuh) batches are decompressed on the GPU into a scratch buffer and
+// then decoded like the others; codes 5-7 are rejected.
 // Not handled: records of aborted transactions are delivered (a read_committed consumer would filter them through the
 // .txnindex / abort markers), legacy magic 0/1 message sets are flagged as malformed.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "kta_inflate.cuh"
 
 namespace kta {
 
 constexpr int LOG_HEADER_BYTES = 61;
-// LOGB_COMPRESSED: a codec without a decompressor here (zstd).  LOGB_LZ4 / LOGB_SNAPPY / LOGB_GZIP: the records section must be
-// decompressed first (log_unc_size_kernel + log_decompress_kernel turn such a batch into LOGB_OK).
-enum LogBatchFlags { LOGB_OK = 0, LOGB_SKIP_CONTROL = 1, LOGB_BAD = 2, LOGB_COMPRESSED = 4, LOGB_LZ4 = 8, LOGB_SNAPPY = 16, LOGB_GZIP = 32 };
-constexpr uint32_t LOGB_CODECS = LOGB_LZ4 | LOGB_SNAPPY | LOGB_GZIP;   // batches log_decompress_kernel turns into LOGB_OK
+// LOGB_COMPRESSED: an unknown codec (attributes codes 5-7).  LOGB_LZ4 / LOGB_SNAPPY / LOGB_GZIP / LOGB_ZSTD: the records section
+// must be decompressed first (log_unc_size_kernel, log_zstd_size_kernel + log_decompress_kernel turn such a batch into LOGB_OK).
+enum LogBatchFlags { LOGB_OK = 0, LOGB_SKIP_CONTROL = 1, LOGB_BAD = 2, LOGB_COMPRESSED = 4, LOGB_LZ4 = 8, LOGB_SNAPPY = 16, LOGB_GZIP = 32,
+                     LOGB_ZSTD = 64 };
+constexpr uint32_t LOGB_CODECS = LOGB_LZ4 | LOGB_SNAPPY | LOGB_GZIP | LOGB_ZSTD;   // batches log_decompress_kernel turns into LOGB_OK
 
 __device__ __forceinline__ uint64_t be_u64(const uint8_t *p) {
     uint64_t v = 0;
@@ -83,10 +86,10 @@ __global__ void log_header_kernel(const uint8_t *bytes, int64_t nbytes, const ui
                 bi.max_ts = (int64_t)be_u64(p + 35);
                 bi.log_append_time = (attrs >> 3) & 1u;
                 if (attrs & 0x20u) bi.flags = LOGB_SKIP_CONTROL;
-                else if (codec <= 3) {
-                    bi.flags = codec == 0 ? LOGB_OK : codec == 1 ? LOGB_GZIP : codec == 2 ? LOGB_SNAPPY : LOGB_LZ4;
+                else if (codec <= 4) {
+                    bi.flags = codec == 0 ? LOGB_OK : codec == 1 ? LOGB_GZIP : codec == 2 ? LOGB_SNAPPY : codec == 3 ? LOGB_LZ4 : LOGB_ZSTD;
                     bi.records = count;
-                } else bi.flags = LOGB_COMPRESSED;   // zstd (4) and unassigned codes
+                } else bi.flags = LOGB_COMPRESSED;   // unassigned codes
             }
         }
         if (bi.flags & (LOGB_BAD | LOGB_COMPRESSED | LOGB_CODECS)) atomicOr(error_flags, bi.flags);
@@ -276,6 +279,10 @@ __host__ __device__ LzWalk snappy_walk(const uint8_t *in, uint32_t n, uint8_t *o
     return w;
 }
 
+}  // namespace kta
+#include "kta_zstd.cuh"   // zstd_walk: built on LzWalk and the copy helpers above
+namespace kta {
+
 // gzip: one member (what producers write: the records section is one gzip stream).  The size pass trusts ISIZE; the copy
 // pass is bounded by it and must produce exactly that many bytes.  The CRC32 of the trailer is not verified (like the batch
 // CRC: check.crcs=false).
@@ -315,12 +322,13 @@ __device__ inline LzWalk gzip_walk(const uint8_t *in, uint32_t n, uint8_t *out, 
 }
 
 // thread per batch: the uncompressed size of a compressed batch's records section → slot[b + 1] = bytes its uncompressed
-// image (header + records, rounded up to 16) needs in the scratch buffer (0 for batches that are not compressed)
+// image (header + records, rounded up to 16) needs in the scratch buffer (0 for batches that are not compressed; zstd
+// batches are sized by log_zstd_size_kernel afterwards)
 __global__ void log_unc_size_kernel(const uint8_t *bytes, const LogBatchInfo *info, int64_t nbatches, uint64_t *slot, uint32_t *error_flags) {
     for (int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < nbatches; b += (int64_t)gridDim.x * blockDim.x) {
         const LogBatchInfo bi = info[b];
         uint64_t need = 0;
-        if (bi.flags & LOGB_CODECS) {
+        if (bi.flags & (LOGB_CODECS & ~LOGB_ZSTD)) {
             const uint8_t *in = bytes + bi.off + LOG_HEADER_BYTES;
             const uint32_t n = bi.len - LOG_HEADER_BYTES;
             LzWalk w{0, false};
@@ -338,17 +346,43 @@ __global__ void log_unc_size_kernel(const uint8_t *bytes, const LogBatchInfo *in
     if (blockIdx.x == 0 && threadIdx.x == 0) slot[0] = 0;
 }
 
-// warp per compressed batch: header copy (compression bits cleared, batchLength = uncompressed) + decompressed records into
-// scratch + slot[b]; the batch's info then points there (offsets are relative to `bytes`: the scratch buffer is simply
-// another place in the same address space) and it is an ordinary LOGB_OK batch for the decoder.
-__global__ void __launch_bounds__(128) log_decompress_kernel(const uint8_t *bytes, LogBatchInfo *info, int64_t nbatches, const uint64_t *slot,
-                                                             uint8_t *scratch, uint32_t *error_flags) {
-    __shared__ InfWork inf_work[4];   // Huffman tables of the warp's gzip batch
+// warp per zstd batch (the sequence tables live in shared memory), after log_unc_size_kernel: slot[b + 1] as there.  A frame
+// that states its content size is taken at that size within what its blocks can hold (the copy pass must then produce
+// exactly that much); a frame without one is walked: literal section sizes plus decoded match lengths, no copies.
+__global__ void __launch_bounds__(128) log_zstd_size_kernel(const uint8_t *bytes, const LogBatchInfo *info, int64_t nbatches, uint64_t *slot,
+                                                            uint32_t *error_flags) {
+    __shared__ ZstdWork zstd_work[4];
     const int lane = threadIdx.x & 31;
     const int64_t gw = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, gs = ((int64_t)gridDim.x * blockDim.x) >> 5;
     for (int64_t b = gw; b < nbatches; b += gs) {
         const LogBatchInfo bi = info[b];
-        if (!(bi.flags & LOGB_CODECS)) continue;
+        if (bi.flags != LOGB_ZSTD) continue;
+        const LzWalk w = zstd_walk<false>(bytes + bi.off + LOG_HEADER_BYTES, bi.len - LOG_HEADER_BYTES, nullptr, 0, zstd_work[threadIdx.x >> 5],
+                                          lane, true);
+        if (lane == 0) {
+            uint64_t need = 0;
+            if (!w.ok || w.out_len > 0x7fffff00ull || (uint64_t)bi.records * 7u > w.out_len) atomicOr(error_flags, (uint32_t)LOGB_BAD);
+            else need = ((uint64_t)LOG_HEADER_BYTES + w.out_len + 15u) & ~15ull;
+            slot[b + 1] = need;
+        }
+    }
+}
+
+// warp per compressed batch: header copy (compression bits cleared, batchLength = uncompressed) + decompressed records into
+// scratch + slot[b]; the batch's info then points there (offsets are relative to `bytes`: the scratch buffer is simply
+// another place in the same address space) and it is an ordinary LOGB_OK batch for the decoder.
+// ZSTD: the zstd batches, with their larger tables (ZstdWork) in shared memory; otherwise the LZ4 / Snappy / gzip batches, so
+// that those keep the registers and shared memory of a kernel without zstd (twice the blocks per SM, measured 1.5x the rate).
+template <bool ZSTD>
+__global__ void __launch_bounds__(128) log_decompress_kernel(const uint8_t *bytes, LogBatchInfo *info, int64_t nbatches, const uint64_t *slot,
+                                                             uint8_t *scratch, uint32_t *error_flags) {
+    using Work = typename std::conditional<ZSTD, ZstdWork, InfWork>::type;
+    __shared__ Work work[4];   // Huffman / FSE tables of the warp's gzip or zstd batch
+    const int lane = threadIdx.x & 31;
+    const int64_t gw = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, gs = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t b = gw; b < nbatches; b += gs) {
+        const LogBatchInfo bi = info[b];
+        if (ZSTD ? bi.flags != LOGB_ZSTD : !(bi.flags & (LOGB_CODECS & ~LOGB_ZSTD))) continue;
         const uint64_t need = slot[b + 1] - slot[b];
         uint8_t *dst = scratch + slot[b];
         if (need < (uint64_t)LOG_HEADER_BYTES) {             // the size pass rejected it
@@ -357,9 +391,19 @@ __global__ void __launch_bounds__(128) log_decompress_kernel(const uint8_t *byte
         }
         const uint8_t *src = bytes + bi.off;
         const uint64_t cap = need - LOG_HEADER_BYTES;
-        const LzWalk w = bi.flags == LOGB_LZ4    ? lz4_frame_walk<true>(src + LOG_HEADER_BYTES, bi.len - LOG_HEADER_BYTES, dst + LOG_HEADER_BYTES, cap, lane)
-                         : bi.flags == LOGB_GZIP ? gzip_walk(src + LOG_HEADER_BYTES, bi.len - LOG_HEADER_BYTES, dst + LOG_HEADER_BYTES, cap, inf_work[threadIdx.x >> 5], lane)
-                                                 : snappy_walk<true>(src + LOG_HEADER_BYTES, bi.len - LOG_HEADER_BYTES, dst + LOG_HEADER_BYTES, cap, lane);
+        const uint8_t *in = src + LOG_HEADER_BYTES;
+        const uint32_t n = bi.len - LOG_HEADER_BYTES;
+        uint8_t *out = dst + LOG_HEADER_BYTES;
+        LzWalk w;
+        if constexpr (ZSTD) {
+            // the records section must come out at exactly the size pass's length (the slot is that, rounded up to 16)
+            w = zstd_walk<true>(in, n, out, cap, work[threadIdx.x >> 5], lane);
+            w.ok = w.ok && ((LOG_HEADER_BYTES + w.out_len + 15u) & ~15ull) == need;
+        } else {
+            w = bi.flags == LOGB_LZ4    ? lz4_frame_walk<true>(in, n, out, cap, lane)
+              : bi.flags == LOGB_GZIP ? gzip_walk(in, n, out, cap, work[threadIdx.x >> 5], lane)
+                                      : snappy_walk<true>(in, n, out, cap, lane);
+        }
         for (int i = lane; i < LOG_HEADER_BYTES; i += 32) dst[i] = src[i];
         __syncwarp();
         if (lane == 0) {

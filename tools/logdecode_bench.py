@@ -9,7 +9,7 @@ from kafka_topic_analyzer_b200._native import lib, check
 
 P, N, VM = 16, 8_000_000, int(sys.argv[1]) if len(sys.argv) > 1 else 256
 BR = int(sys.argv[2]) if len(sys.argv) > 2 else 56   # ~16 KB batches (the producer default batch.size) at 256 B values
-CODEC = sys.argv[3] if len(sys.argv) > 3 else None   # gzip | lz4 | snappy: every batch's records section compressed (zlib / pyarrow) on the host
+CODEC = sys.argv[3] if len(sys.argv) > 3 else None   # gzip | lz4 | snappy | zstd: every batch's records section compressed (zlib / pyarrow) on the host
 if CODEC:
     N = 2_000_000
 
@@ -25,10 +25,12 @@ def compress_segment(seg: np.ndarray, codec: str) -> np.ndarray:
             import zlib
             c = zlib.compressobj(6, zlib.DEFLATED, 31)
             body = c.compress(raw[pos + 61:pos + 12 + bl]) + c.flush()
+        elif codec == "zstd":   # level 3, librdkafka's default
+            body = pa.Codec("zstd", compression_level=3).compress(raw[pos + 61:pos + 12 + bl], asbytes=True)
         else:
             body = pa.compress(raw[pos + 61:pos + 12 + bl], codec=codec, asbytes=True)
         hdr[8:12] = (49 + len(body)).to_bytes(4, "big")
-        hdr[22] |= {"gzip": 1, "snappy": 2, "lz4": 3}[codec]
+        hdr[22] |= {"gzip": 1, "snappy": 2, "lz4": 3, "zstd": 4}[codec]
         out += hdr + body
         pos += 12 + bl
     return np.frombuffer(bytes(out), dtype=np.uint8)

@@ -15,21 +15,28 @@ which = sys.argv[1:] or ["counters", "hll", "exact", "ragged", "ring", "log", "l
 
 
 def compress_segment(seg, b0=0):
-    """every batch of an uncompressed segment re-written with its records section compressed: gzip, LZ4, Snappy in turn"""
+    """every batch of an uncompressed segment re-written with its records section compressed: gzip, LZ4, Snappy, zstd in turn
+    (zstd with and without a content size in the frame header)"""
     import zlib
     import pyarrow as pa
     raw, out, pos, b = seg.tobytes(), bytearray(), 0, b0
     while pos + 61 <= len(raw):
         bl = int.from_bytes(raw[pos + 8:pos + 12], "big", signed=True)
         hdr, body = bytearray(raw[pos:pos + 61]), raw[pos + 61:pos + 12 + bl]
-        codec = ("gzip", "lz4", "snappy")[b % 3]
+        codec = ("gzip", "lz4", "snappy", "zstd", "zstd-nofcs")[b % 5]
         if codec == "gzip":
             c = zlib.compressobj(6, zlib.DEFLATED, 31)
             body = c.compress(body) + c.flush()
+        elif codec.startswith("zstd"):
+            body = pa.Codec("zstd", compression_level=3).compress(body, asbytes=True)
+            if codec == "zstd-nofcs":
+                import zstd_codec
+                body = zstd_codec.without_fcs(body)
+            codec = "zstd"
         else:
             body = pa.compress(body, codec=codec, asbytes=True)
         hdr[8:12] = (49 + len(body)).to_bytes(4, "big")
-        hdr[22] |= {"gzip": 1, "snappy": 2, "lz4": 3}[codec]
+        hdr[22] |= {"gzip": 1, "snappy": 2, "lz4": 3, "zstd": 4}[codec]
         out += hdr + body
         pos += 12 + bl
         b += 1
@@ -47,7 +54,7 @@ for name in which:
         with kta.KtaEngine(P, count_alive_keys=True, hll_precision=10, device=0, now=NOW, alive_table_kib=1) as e:
             per = n // P
             segs = [(p, synth.encode_segment(spec, p, 0, per, batch_records=100)) for p in range(P)]
-            if name == "logz":   # gzip / LZ4 / Snappy batches: the decompressors run first
+            if name == "logz":   # gzip / LZ4 / Snappy / zstd batches: the decompressors run first
                 segs = [(p, compress_segment(s, p)) for p, s in segs]
             e.push_log_segments(segs)
             e.finalize()
